@@ -24,6 +24,11 @@ padding, generator seed 1234), seeded random-init weights (checkpoints are unrea
 `cpu_baseline`: the reference on the box's host cores, on a bounded sample (N=1, rank 0 only): the unmodified
            reference when baseline/_ref is present (kind "reference"), else the oracle port (kind "port").
 Only the baseline legs and --impl reference import oracle/ or baseline/_ref; the product path never does.
+
+--dump-outputs DIR writes what the last timed step returned, the per-sequence mean representations [batch, E], as
+DIR/mean_representations.npy (float32; above 64 MB a fixed seeded sample of its rows).  Tokens (seed 1234) and weights
+(seed 0, or the local checkpoint) are the same on every run with the same arguments, so two builds can be compared
+output for output.
 """
 from __future__ import annotations
 
@@ -250,6 +255,24 @@ def timed(fn, reps, warm):
     return a.elapsed_time(b) / reps
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """arrays {name: tensor} -> path/<name>.npy in float32, together at most DUMP_BYTES: a larger array keeps a fixed
+    seeded sample of its rows (leading dimension)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    cap = DUMP_BYTES // len(arrays)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        row_bytes = t[0].numel() * 4
+        if t.numel() * 4 > cap:
+            keep = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:cap // row_bytes]
+            t = t[keep.sort().values.to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
+
+
 def extra_configs(dev, peaks):
     """BASELINE.json configs[3] and configs[4] on this GPU (N=1): seeded random init built on the device."""
     from esm_b200 import pretrained
@@ -311,7 +334,10 @@ def main():
     ap.add_argument("--cpu-baseline-seqs", type=int, default=4)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip configs[3]/[4] and the GPU eager baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's result as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -361,12 +387,14 @@ def main():
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
     for _ in range(args.steps):
-        step_device()
+        mean = step_device()
     ev1.record()
     torch.cuda.synchronize()
     barrier()
     ms_total = ev0.elapsed_time(ev1)
     launches = lib.esmb200_launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"mean_representations": mean})
 
     # ---- per-kernel pass: the same step with every launch bracketed by events (breaks PDL overlap, so it is separate)
     prof_steps = min(2, args.steps)

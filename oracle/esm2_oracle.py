@@ -84,6 +84,49 @@ def transformer_layer(x: torch.Tensor, sd: Dict[str, torch.Tensor], pre: str, nu
     return x, probs
 
 
+class TransformerLayer(torch.nn.Module):
+    """esm/modules.py:84-142 as a module: the reference's parameter names, `use_rotary_embeddings` and forward signature
+    ((T, B, E) in and out, per-head probabilities (H, B, T, T) when need_head_weights), evaluated by transformer_layer().
+    It gives tests the reference's layer seam (what esm_b200.integration.patch_reference substitutes) without the
+    reference package."""
+
+    use_rotary_embeddings = True
+
+    def __init__(self, embed_dim: int, attention_heads: int):
+        super().__init__()
+        E, nn = embed_dim, torch.nn
+        self.self_attn = nn.Module()
+        for name in ("q_proj", "k_proj", "v_proj", "out_proj"):
+            setattr(self.self_attn, name, nn.Linear(E, E))
+        self.self_attn.num_heads = attention_heads
+        self.self_attn.bias_k = None
+        self.self_attn.rot_emb = nn.Module()
+        self.self_attn.rot_emb.register_buffer("inv_freq", torch.zeros(E // attention_heads // 2))
+        self.self_attn_layer_norm = nn.LayerNorm(E)
+        self.fc1 = nn.Linear(E, 4 * E)
+        self.fc2 = nn.Linear(4 * E, E)
+        self.final_layer_norm = nn.LayerNorm(E)
+
+    def forward(self, x, self_attn_mask=None, self_attn_padding_mask=None, need_head_weights=False):
+        assert self_attn_mask is None
+        y, p = transformer_layer(x.transpose(0, 1), self.state_dict(), "", self.self_attn.num_heads,
+                                 self_attn_padding_mask, need_head_weights)
+        return y.transpose(0, 1), (p.transpose(0, 1) if need_head_weights else None)
+
+
+def layer_modules(sd: Dict[str, torch.Tensor], num_layers: int, num_heads: int):
+    """The layers of a state dict as TransformerLayer modules (on the device and in the dtype of `sd`)."""
+    E = sd["embed_tokens.weight"].shape[1]
+    layers = []
+    for i in range(num_layers):
+        pre = f"layers.{i}."
+        with torch.device("meta"):  # no initialisation: every tensor is assigned from `sd`
+            m = TransformerLayer(E, num_heads)
+        m.load_state_dict({k[len(pre):]: v for k, v in sd.items() if k.startswith(pre)}, strict=True, assign=True)
+        layers.append(m)
+    return layers
+
+
 def embed(tokens: torch.Tensor, sd: Dict[str, torch.Tensor], token_dropout: bool = True) -> torch.Tensor:
     """esm/model/esm2.py:82-95 — embedding gather, <mask> rows zeroed and x * 0.88 / (1 - n_mask/n_nonpad) when
     token_dropout (active at inference), pad rows zeroed."""
@@ -121,8 +164,10 @@ def contact_head(tokens: torch.Tensor, attentions: torch.Tensor, sd: Dict[str, t
 @torch.no_grad()
 def esm2_forward(sd: Dict[str, torch.Tensor], num_layers: int, num_heads: int, tokens: torch.Tensor,
                  repr_layers: Iterable[int] = (), need_head_weights: bool = False, return_contacts: bool = False,
-                 token_dropout: bool = True):
-    """esm/model/esm2.py:77-144 — same result dict as ESM2.forward."""
+                 token_dropout: bool = True, layers=None):
+    """esm/model/esm2.py:77-144 — same result dict as ESM2.forward.  `layers`: modules with the reference's
+    TransformerLayer interface (layer_modules()) that run the layer loop in its (T, B, E) layout, as esm2.py:105-121
+    does; by default the functional transformer_layer() runs it."""
     if return_contacts:
         need_head_weights = True
     repr_layers = set(repr_layers)
@@ -134,7 +179,11 @@ def esm2_forward(sd: Dict[str, torch.Tensor], num_layers: int, num_heads: int, t
     mask = pad if bool(pad.any()) else None
     probs = []
     for i in range(num_layers):
-        x, p = transformer_layer(x, sd, f"layers.{i}.", num_heads, mask, need_head_weights)
+        if layers is None:
+            x, p = transformer_layer(x, sd, f"layers.{i}.", num_heads, mask, need_head_weights)
+        else:
+            y, p = layers[i](x.transpose(0, 1), self_attn_padding_mask=mask, need_head_weights=need_head_weights)
+            x, p = y.transpose(0, 1), (p.transpose(0, 1) if need_head_weights else None)
         if (i + 1) in repr_layers:
             hidden[i + 1] = x
         if need_head_weights:
